@@ -1,4 +1,4 @@
-"""The reference's training / eval step driven through the reference's OWN modules (baseline/_ref mirror of the
+"""The reference's training / eval step driven through the reference's OWN modules (oracle/_ref mirror of the
 checkout: models.preprocess.AugmentMelSTFT, models.mn.model.get_model, models.dymn.model.get_model, helpers.utils.mixup)
 -- measurement infrastructure for bench.py's reference arms, never imported by the product.
 
@@ -18,7 +18,7 @@ import torch
 import torch.nn.functional as F
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.path.join(HERE, "_ref")
+REF = os.path.join(os.path.dirname(HERE), "oracle", "_ref")
 
 
 def available():

@@ -47,7 +47,31 @@ def parse():
     ap.add_argument("--sync-readback", action="store_true",
                     help="e2e loop: read the loss back with a blocking .cpu() after every step instead of the pipelined LossReader")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel eagerly instead of replaying a CUDA graph")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (rank 0), for comparing two builds")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Write {name: device tensor} as DIR/<name>.npy in float32 / float64, at most DUMP_MAX_BYTES in all.  A larger
+    tensor is cut to a fixed sample (seeded indices, sorted), the same for every run with the same arguments."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    budget = DUMP_MAX_BYTES // max(len(arrays), 1)
+    for name, t in arrays.items():
+        t = t.detach().reshape(-1)
+        t = t.double() if t.dtype == torch.float64 else t.float()
+        cap = budget // t.element_size()
+        if t.numel() > cap:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:cap].sort().values
+            t = t[idx.to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
 
 
 # ----------------------------------------------------------------------------------------------- clocks
@@ -102,7 +126,7 @@ def _synth_batch(batch, seed):
 
 
 def cpu_reference_step_factory(batch, model="mn10"):
-    """One training step of the reference on the host: the reference's OWN modules from the baseline/_ref mirror when it
+    """One training step of the reference on the host: the reference's OWN modules from the oracle/_ref mirror when it
     is present (kind "reference"), else the oracle port of the same algorithm (kind "port").  Same step as the GPU arm:
     mel + mixup + forward + hard/distillation BCE with the unknown-teacher mask + backward + Adam."""
     from baseline import ref_step
@@ -204,7 +228,7 @@ def run_reference_arm(args):
     if rank != 0:
         return
     value, s_per_step, cores, b, kind = time_cpu_reference(args.cpu_baseline_batch, args.steps, args.warmup, model=args.model)
-    what = "the reference's own modules (baseline/_ref mirror)" if kind == "reference" else "oracle port of the reference modules"
+    what = "the reference's own modules (oracle/_ref mirror)" if kind == "reference" else "oracle port of the reference modules"
     sample = f"{args.steps} steps x {b} clips ({args.warmup} warm-up), same training step as the GPU arm, fp32, {what}"
     line = {"impl": "reference", "metric": METRIC if args.model == "mn10" else f"clips/sec (10s@32kHz) {args.model}_as fwd+bwd",
             "value": value, "unit": "clips/s", "n_gpus": args.gpus,
@@ -252,7 +276,7 @@ def time_reference_gpu(model, mode, B, steps, warmup, dev, amp, world, seed):
 def gpu_baseline_entry(model, mode, B, steps, warmup, dev, amp, world, seed):
     from baseline import ref_step
     if not ref_step.available():
-        return {"unavailable": "baseline/_ref (mirror of the reference checkout, made by baseline/make_ref.py) is not present"}
+        return {"unavailable": "oracle/_ref (mirror of the reference checkout, made by oracle/make_ref.py) is not present"}
     try:
         ms, gib = time_reference_gpu(model, mode, B, steps, warmup, dev, amp, world, seed)
     except torch.cuda.OutOfMemoryError:
@@ -260,7 +284,7 @@ def gpu_baseline_entry(model, mode, B, steps, warmup, dev, amp, world, seed):
         return {"unavailable": f"reference modules ran out of memory at batch {B}/GPU", "amp": amp}
     return {"value": world * B * steps / (ms * 1e-3), "unit": "clips/s", "ms_per_step": ms / steps, "steps": steps,
             "amp": amp, "batch_per_gpu": B, "peak_mem_gib": round(gib, 1),
-            "what": "the reference's own nn.Modules (baseline/_ref mirror) through stock PyTorch: cuFFT + cuDNN + cuBLAS, "
+            "what": "the reference's own nn.Modules (oracle/_ref mirror) through stock PyTorch: cuFFT + cuDNN + cuBLAS, "
                     "cudnn.benchmark, " + ("fp32 params / TF32 convolutions (PyTorch defaults)" if amp == "none" else "torch.autocast(bfloat16)")
                     + (", DistributedDataParallel" if world > 1 else "") + "; same synthetic batch and loop body "
                     "(ex_audioset.py:135-199 incl. its 3 loss read-backs per step)"}
@@ -463,6 +487,7 @@ def run_ours(args):
             def step(self, w, y_, t_, k_=None):
                 with torch.no_grad():
                     logits, _ = model(mel(w).unsqueeze(1))
+                self.logits = logits
                 return logits[:, :2].double().sum(0)             # tiny device result read back in the e2e loop
         trainer = _Eval()
     import numpy as np
@@ -522,6 +547,13 @@ def run_ours(args):
         host_ms = (time.perf_counter() - h0) * 1e3 / args.steps      # time the host needs to ENQUEUE one step
         barrier()
     ms = e0.elapsed_time(e1)
+    # what the last timed step computed: its [label, distillation] loss and the parameters its Adam update wrote (train),
+    # or the logits (eval).  Copied out now: the steps below keep training the same model.  Compare parameters with a
+    # tolerance: Adam turns the reduction-order noise of small gradients into differences of a fraction of lr per step
+    # (two runs of one build, mn10, 10 timed steps, one B200: up to 8e-3, 99.9 % within 2.4e-3; the loss within 1e-5)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": loss, "params": real.flat_p} if args.mode == "train"
+                     else {"logits": trainer.logits})
     if world > 1:
         t = torch.tensor([ms], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -646,7 +678,7 @@ def run_ours(args):
             line["cpu_baseline"] = {"value": v, "unit": "clips/s", "cores": cores, "kind": kind,
                                     "sample": f"2 steps x {cb} clips (1 warm-up), same training step (mixup, hard + "
                                               "distillation loss with the unknown-teacher mask, Adam), fp32, "
-                                              + ("the reference's own modules (baseline/_ref mirror)" if kind == "reference"
+                                              + ("the reference's own modules (oracle/_ref mirror)" if kind == "reference"
                                                  else "oracle port of the reference modules") + " on the host cores"}
     # ---- the reference's own GPU path on the same device(s): cuFFT / cuDNN / cuBLAS through the unmodified modules
     gb = None

@@ -3,7 +3,7 @@
 package (`--side ours`: `dropin/` shadows `models.*`, `helpers.utils`, `datasets.audioset`) or against the reference's
 own modules (`--side reference`, used to produce golden numbers on CPU and the cuDNN baseline on GPU).
 
-    python scripts/run_reference_script.py --side ours --ref-root baseline/_ref --log-json out.json \
+    python scripts/run_reference_script.py --side ours --ref-root oracle/_ref --log-json out.json \
         ex_audioset.py -- --train --cuda --pretrained --model_name mn04_as --batch_size 4 --num_workers 0 ...
 
 The script file itself is executed with runpy from `--ref-root`; nothing in it is edited.  What the launcher sets up
@@ -116,7 +116,7 @@ def _install_wandb(log_json):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--side", choices=["ours", "reference"], required=True)
-    ap.add_argument("--ref-root", default=os.path.join(REPO, "baseline", "_ref"))
+    ap.add_argument("--ref-root", default=os.path.join(REPO, "oracle", "_ref"))
     ap.add_argument("--seed", type=int, default=None)
     ap.add_argument("--no-dropout", action="store_true")
     ap.add_argument("--log-json", default=None)
@@ -131,7 +131,7 @@ def main():
     ref_root = os.path.abspath(a.ref_root)
     script = os.path.join(ref_root, a.script)          # an absolute path (a driver under tests/golden/) is taken as is
     if not os.path.isfile(script):
-        raise SystemExit(f"{script} not found (run `python baseline/make_ref.py` where the reference checkout exists)")
+        raise SystemExit(f"{script} not found (run `python oracle/make_ref.py` where the reference checkout exists)")
     rest = a.rest[1:] if a.rest and a.rest[0] == "--" else a.rest
 
     # import resolution: the script's own directory is NOT put first (runpy.run_path does not do it), so `models.*`

@@ -170,8 +170,7 @@ def golden_script():
         assert r.returncode == 0, r.stderr[-3000:]
         sd = torch.load(ck, map_location="cpu")
         res = {"args": R.SCRIPT_ARGS, "env": R.SCRIPT_ENV, "epochs": R.read_log(log), "final_state": state_digest(sd)}
-        r = R.run_script(wd, "reference", "inference.py", ["--model_name", "mn10_as", "--audio_path",
-                                                          os.path.join(R.ref_root(), "resources", "metro_station-paris.wav")],
+        r = R.run_script(wd, "reference", "inference.py", ["--model_name", "mn10_as", "--audio_path", R.WAV],
                          env, no_dropout=False)
         assert r.returncode == 0, r.stderr[-3000:]
         rows = re.findall(r"^(.+): (\d\.\d{3})$", r.stdout, flags=re.M)
@@ -196,7 +195,7 @@ def golden_script_f4():
     import tempfile
     from tests import refscripts as R
     os.chdir(REPO)
-    wav = os.path.join(R.ref_root(), "resources", "metro_station-paris.wav")
+    wav = R.WAV
     res = {"window_s": 2.0, "hop_s": 1.0, "ensemble": ["mn04_as", "mn10_as"]}
     with tempfile.TemporaryDirectory() as wd:
         env = R.make_workdir(wd, checkpoints=("mn04_as", "mn10_as"))

@@ -20,21 +20,25 @@ SCRIPT_ARGS = ["--train", "--pretrained", "--model_name", "mn04_as", "--batch_si
                "--ramp_down_len", "4", "--last_lr_value", "0.1", "--max_lr", "0.0004"]
 
 
+# recording and AudioSet label table the scripts read (resources/, metadata/ of the original project; the recording is
+# stored resampled to 32 kHz, the rate every consumer reads it at, 16-bit; the goldens were produced from this file)
+WAV = os.path.join(REPO, "tests", "golden", "metro_station-paris.wav")
+METADATA = os.path.join(REPO, "tests", "golden", "metadata")
+
+
 def ref_root():
-    for p in (os.path.join(REPO, "baseline", "_ref"), "/root/reference"):
-        if os.path.isfile(os.path.join(p, "ex_audioset.py")):
-            return p
-    return None
+    """the mirror of the original EfficientAT project that build() makes (oracle/make_ref.py), or None"""
+    p = os.path.join(REPO, "oracle", "_ref")
+    return p if os.path.isfile(os.path.join(p, "ex_audioset.py")) else None
 
 
 def make_workdir(path, checkpoints=("mn04_as",), env=None):
     """-> env dict for the subprocess.  `checkpoints`: release names whose synthetic state (tests/util.build_model:
     seeded weights + calibrated BatchNorm buffers) is stored under the reference's file name in resources/."""
     from tests.util import build_model
-    root = ref_root()
     os.makedirs(os.path.join(path, "resources"), exist_ok=True)
-    if root is not None and not os.path.exists(os.path.join(path, "metadata")):
-        shutil.copytree(os.path.join(root, "metadata"), os.path.join(path, "metadata"))
+    if not os.path.exists(os.path.join(path, "metadata")):
+        shutil.copytree(METADATA, os.path.join(path, "metadata"))
     for name in checkpoints:
         m = build_model(name.split("_")[0])
         torch.save({k: v.clone() for k, v in m.state_dict().items()}, os.path.join(path, "resources", RELEASE_FILE[name]))

@@ -1,7 +1,7 @@
 """SURVEY.md section 8 row f1: the reference's OWN entry scripts, byte-for-byte unchanged, running on this package.
 
-`baseline/_ref/` (mirror of the reference checkout made by baseline/make_ref.py; git-ignored, travels to the GPU box)
-supplies ex_audioset.py / inference.py; scripts/run_reference_script.py executes them with `dropin/` first on the
+`oracle/_ref/` (mirror of the reference checkout made by build() through oracle/make_ref.py; git-ignored, travels with
+the working tree) supplies ex_audioset.py / inference.py; scripts/run_reference_script.py executes them with `dropin/` first on the
 import path, so `models.mn.model.get_model`, `models.preprocess.AugmentMelSTFT`, `helpers.utils` and `datasets.audioset`
 resolve to this repository.  The expected numbers (tests/golden/script_mn04.json) were produced by the same launcher
 with `--side reference` on CPU: the reference's own modules under the same scripts, seeds, synthetic clips and
@@ -19,7 +19,8 @@ from tests.util import report, GOLDEN
 
 pytestmark = pytest.mark.gpu
 
-needs_ref = pytest.mark.skipif(R.ref_root() is None, reason="baseline/_ref (mirror of the reference checkout) not present")
+needs_ref = pytest.mark.skipif(R.ref_root() is None, reason="oracle/_ref (mirror of the reference checkout that build() "
+                               "makes) not present")
 
 
 def _golden():
@@ -73,15 +74,14 @@ def test_ex_audioset_train_runs_unchanged_and_matches_reference_run(tmp_path):
 
 @needs_ref
 def test_inference_py_runs_unchanged_and_prints_reference_labels(tmp_path):
-    """BASELINE.json configs[0]: inference.py --cuda on resources/metro_station-paris.wav with a (synthetic) mn10_as
+    """BASELINE.json configs[0]: inference.py --cuda on the recording fixture (golden/metro_station-paris.wav) with a (synthetic) mn10_as
     checkpoint loaded through the reference's release-file path.  The ten printed labels must be the reference run's,
     in order, with probabilities within 2e-3 (the script prints 3 decimals; the reference run was fp32 on CPU, this
     one runs under the script's `autocast`, which this package's fp32 kernels ignore)."""
     g = _golden()
     wd = str(tmp_path)
     env = R.make_workdir(wd, checkpoints=("mn10_as",))
-    wav = os.path.join(R.ref_root(), "resources", "metro_station-paris.wav")
-    r = R.run_script(wd, "ours", "inference.py", ["--cuda", "--model_name", "mn10_as", "--audio_path", wav], env,
+    r = R.run_script(wd, "ours", "inference.py", ["--cuda", "--model_name", "mn10_as", "--audio_path", R.WAV], env,
                      no_dropout=False)
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-4000:]
     rows = re.findall(r"^(.+): (\d\.\d{3})$", r.stdout, flags=re.M)

@@ -19,7 +19,8 @@ from tests import refscripts as R
 from tests.util import GOLDEN, build_model, golden, net_inputs, report
 
 pytestmark = pytest.mark.gpu
-needs_ref = pytest.mark.skipif(R.ref_root() is None, reason="baseline/_ref (mirror of the reference checkout) not present")
+needs_ref = pytest.mark.skipif(R.ref_root() is None, reason="oracle/_ref (mirror of the reference checkout that build() "
+                               "makes) not present")
 
 
 def _golden():
@@ -28,7 +29,7 @@ def _golden():
 
 
 def _wav():
-    return os.path.join(R.ref_root(), "resources", "metro_station-paris.wav")
+    return R.WAV
 
 
 def _same_ranking(got, want, tol):
@@ -94,7 +95,6 @@ def _shim_loader():
     return load
 
 
-@needs_ref
 @pytest.mark.parametrize("which", ["windowed_mn10", "windowed_ensemble"])
 def test_native_batched_tagger_matches_reference_eatagger(tmp_path, monkeypatch, which):
     """efficientat_b200.windowed.EATagger: all 9 windows through ONE mel launch and ONE forward at batch 9, top-k on the
